@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - TensorProto encode+decode throughput on B200 (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c5] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4|c5] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic requests: ONE ``b200tfs_encode_requests`` call
 over the batch's PredictRequests (device tensors -> wire arena) and ONE decode call over the batch's
@@ -628,6 +628,46 @@ class DeviceBatch:
         self.lib.b200tfs_destroy(self.ctx)
 
 
+DUMP_VALUES = 7 << 20       # values kept per dumped stream: two float32 streams stay under 64 MiB
+
+
+def dump_outputs(db: DeviceBatch, s, out_dir):
+    """Write what the step on ring slot `s` handed its caller to out_dir as .npy files: `request_wire` (the bytes of every
+    encoded request, request after request, as float32 byte values), `request_wire_len` (float64, one per request) and
+    `response_<key>` (every decoded tensor as float32, response after response).  A stream of more than DUMP_VALUES values
+    keeps a fixed sample of its positions (np.random.default_rng(0) over the stream's length), so runs with the same
+    arguments dump the same positions and two builds compare value for value.  Every array is finite: the NaNs the
+    workloads plant in their inputs (the sNaN probe) come back decoded, so `response_<key>` holds 0 at a non-finite
+    output and `response_<key>_nonfinite` (float64, one row per such output) its flat index and exact bit pattern."""
+    os.makedirs(out_dir, exist_ok=True)
+    st, n, wl = db.sets[s % db.slots], db.n, db.wl
+    db.encode_results(s)
+    rec = [(int(st["rec_off"][j]), int(st["rec_len"][j])) for j in range(n)]
+    np.save(os.path.join(out_dir, "request_wire_len.npy"), np.array([ln for _, ln in rec], dtype=np.float64))
+    key, rx = db.host_resp[wl.seed_of(db.lo)] if n else ("y", np.zeros(0, np.float32))
+    out_dt = np.dtype(wl.np_dtype if wl.out_dtype is not None else np.float32)
+    streams = (("request_wire", np.dtype(np.uint8), [(st["arena"] + o, ln) for o, ln in rec], None),
+               ("response_" + key, out_dt, [(st["dst"] + j * db.dst_stride, db.dst_bytes) for j in range(n)], (n,) + rx.shape))
+    for name, dt, pieces, shape in streams:
+        total = sum(nb // dt.itemsize for _, nb in pieces)
+        pos = np.unique(np.random.default_rng(0).integers(0, total, size=DUMP_VALUES)) if total > DUMP_VALUES else None
+        vals, start = [], 0
+        for ptr, nb in pieces:
+            cnt = nb // dt.itemsize
+            take = slice(None) if pos is None else pos[np.searchsorted(pos, start): np.searchsorted(pos, start + cnt)] - start
+            if pos is None or len(take):
+                vals.append(db.download(ptr, nb).view(dt)[take])
+            start += cnt
+        raw = np.concatenate(vals) if vals else np.zeros(0, dt)
+        arr = raw.astype(np.float32)
+        if shape:
+            bad = np.flatnonzero(~np.isfinite(arr))
+            bits = raw.view(np.dtype("u%d" % dt.itemsize))[bad]
+            np.save(os.path.join(out_dir, name + "_nonfinite.npy"), np.stack([bad, bits], axis=1).astype(np.float64).reshape(-1, 2))
+            arr[bad] = 0.0
+        np.save(os.path.join(out_dir, name + ".npy"), arr.reshape(shape) if pos is None and shape else arr)
+
+
 # ------------------------------------------------------------------------------------------------
 # e2e: the same hot path through the host-buffer C-ABI entry points (what a client binds)
 # ------------------------------------------------------------------------------------------------
@@ -787,7 +827,7 @@ def ncu_traffic(workload, n_on_rank=None):
 # ------------------------------------------------------------------------------------------------
 # one workload on this rank -> the pieces of the bench line
 # ------------------------------------------------------------------------------------------------
-def run_workload(wl: Workload, world: World, steps, warmup, e2e_steps, full_verify, sampler=None, e2e=True):
+def run_workload(wl: Workload, world: World, steps, warmup, e2e_steps, full_verify, sampler=None, e2e=True, dump_dir=None):
     peak, peak_src = peaks()
     db = DeviceBatch(wl, world.local_rank, world.size, world.rank)
     assert db.footprint > L2_BYTES or db.n == 0, "the batch ring must exceed L2"
@@ -827,6 +867,8 @@ def run_workload(wl: Workload, world: World, steps, warmup, e2e_steps, full_veri
     world.barrier()
     launches = (db.launches() - l0) if mode == "eager" else per_replay * (steps // db.slots) + (db.graphs["step_rem"][1] if steps % db.slots else 0)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if dump_dir and world.rank == 0:
+        dump_outputs(db, steps - 1, dump_dir)                   # the last timed step ran on slot (steps - 1) % slots
     ms_max = world.max(ms)
     payload = world.sum(float(db.payload_bytes() * steps))
     value = payload / (ms_max * 1e-3) / 1e9
@@ -1198,6 +1240,8 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="default c2 run only: skip the short c3 / c4 / c5 passes reported under `workloads`")
     ap.add_argument("--verify", default="full", choices=["full", "sample"], help="parity check after the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the request wires and decoded tensors of the last timed step "
+                                                          "(rank 0's share; a fixed sample of a large batch) to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":   # CPU only: rank 0 works alone, nobody needs a process group
         run_reference(args)
@@ -1209,7 +1253,8 @@ def main():
     warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload](args.batch or None)
     sampler = ClockSampler(world.local_rank)
-    res = run_workload(wl, world, args.steps, warmup, args.e2e_steps, full_verify=(args.verify == "full"), sampler=sampler)
+    res = run_workload(wl, world, args.steps, warmup, args.e2e_steps, full_verify=(args.verify == "full"), sampler=sampler,
+                       dump_dir=args.dump_outputs)
     extras = {}
     if args.workload == "c2":
         if not args.no_extra:

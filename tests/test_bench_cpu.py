@@ -7,7 +7,6 @@ import subprocess
 import sys
 
 import numpy as np
-import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, REPO)
@@ -63,23 +62,6 @@ def test_cpu_baseline_leg_runs_the_unmodified_reference():
         t, origin = ref_loader.load()
         assert "reference" in origin and not t.__file__.startswith(os.path.join(REPO, "min-tfs-client_b200"))
     assert bench.cpu_c_oracle(1)["value"] > r["value"]          # plain C beats per-element Python
-
-
-def test_staged_reference_archive_matches_the_checkout():
-    """baseline/_ref/min_tfs_client_reference.zip holds the three reference modules byte for byte (when both are present)."""
-    import hashlib
-    import zipfile
-
-    from baseline import ref_loader, stage_reference
-
-    if not (os.path.isdir(ref_loader.REF_DIR) and os.path.exists(ref_loader.ZIP)):
-        pytest.skip("needs the reference checkout and the staged archive")
-    with zipfile.ZipFile(ref_loader.ZIP) as z:
-        manifest = json.loads(z.read("MANIFEST.json"))
-        for f in stage_reference.FILES:
-            with open(os.path.join(ref_loader.REF_DIR, f), "rb") as fh:
-                blob = fh.read()
-            assert z.read("min_tfs_client/" + f) == blob and manifest[f] == hashlib.sha256(blob).hexdigest()
 
 
 def test_host_cores_is_sane():

@@ -1,7 +1,5 @@
-"""The schema modules written by tools/gen_pb2.py against (a) the reference's own .proto files when
-/root/reference is present (build container) and (b) the reference's dtype table / unit-test goldens."""
-import os
-import re
+"""The schema modules written by tools/gen_pb2.py against (a) the field tables of the reference's own .proto files
+(tests/golden/schema.json) and (b) the reference's dtype table / unit-test goldens."""
 
 import numpy as np
 import pytest
@@ -11,7 +9,9 @@ from tensorflow.core.example import example_pb2, feature_pb2
 from tensorflow_serving.apis import classification_pb2, get_model_status_pb2, input_pb2, model_pb2, predict_pb2, regression_pb2
 from tensorflow_serving.util import status_pb2
 
-REF = "/root/reference/protobuf_srcs"
+import golden_util
+
+SCHEMA = golden_util.load("schema.json")
 
 # reference tests/unit/min_tfs_client/types_test.py:7-23
 TEST_TARGETS = [(np.float16, "DT_HALF", 19), (np.float32, "DT_FLOAT", 1), (np.float64, "DT_DOUBLE", 2), (np.int8, "DT_INT8", 6),
@@ -43,27 +43,9 @@ def test_datatype_errors():
         DataType("DT_QINT8")
 
 
-def _proto_fields(path, message):
-    """Tiny tokenizer: {field name: (number, type, repeated, packed)} of one top-level message."""
-    text = re.sub(r"//.*", "", open(path).read())
-    m = re.search(r"message\s+%s\s*\{" % message, text)
-    depth, i, start = 1, m.end(), m.end()
-    while depth:
-        depth += {"{": 1, "}": -1}.get(text[i], 0)
-        i += 1
-    body = text[start:i - 1]
-    body = re.sub(r"message\s+\w+\s*\{[^{}]*\}", "", body)           # drop nested messages
-    body = re.sub(r"oneof\s+\w+\s*\{([^{}]*)\}", r"\1", body)        # flatten oneofs
-    out = {}
-    for rep, typ, name, num, opts in re.findall(r"(repeated\s+)?(map<[^>]+>|[\w.]+)\s+(\w+)\s*=\s*(\d+)\s*(\[[^\]]*\])?\s*;", body):
-        out[name] = (int(num), typ.strip(), bool(rep), "packed = true" in (opts or ""))
-    return out
-
-
 _TYPE = {1: "double", 2: "float", 3: "int64", 4: "uint64", 5: "int32", 8: "bool", 9: "string", 12: "bytes", 13: "uint32"}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present on this box")
 @pytest.mark.parametrize("path,message,cls", [
     ("tensorflow/core/framework/tensor.proto", "TensorProto", tensor_pb2.TensorProto),
     ("tensorflow/core/framework/tensor.proto", "VariantTensorDataProto", tensor_pb2.VariantTensorDataProto),
@@ -92,13 +74,13 @@ _TYPE = {1: "double", 2: "float", 3: "int64", 4: "uint64", 5: "int32", 8: "bool"
     ("tensorflow_serving/util/status.proto", "StatusProto", status_pb2.StatusProto),
 ])
 def test_fields_match_reference_proto(path, message, cls):
-    want = _proto_fields(os.path.join(REF, path), message)
+    want = SCHEMA["messages"][path][message]
     have = {f.name: f for f in cls.DESCRIPTOR.fields}
     assert set(want) == set(have), (sorted(want), sorted(have))
-    for name, (num, typ, rep, packed) in want.items():
+    for name, (num, typ, rep) in want.items():
         f = have[name]
         assert f.number == num, name
-        if typ.startswith("map<"):
+        if typ == "map":
             assert f.message_type.GetOptions().map_entry
             continue
         is_rep = f.is_repeated if hasattr(f, "is_repeated") else f.label == f.LABEL_REPEATED
@@ -111,10 +93,8 @@ def test_fields_match_reference_proto(path, message, cls):
             assert f.message_type.name == typ.split(".")[-1], name
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present on this box")
 def test_datatype_enum_matches_reference_proto():
-    text = re.sub(r"//.*", "", open(os.path.join(REF, "tensorflow/core/framework/types.proto")).read())
-    want = {n: int(v) for n, v in re.findall(r"(DT_\w+)\s*=\s*(\d+)\s*;", text)}
+    want = SCHEMA["DataType"]
     have = {v.name: v.number for v in types_pb2.DataType.DESCRIPTOR.values}
     assert want == have
 
